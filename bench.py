@@ -224,6 +224,30 @@ def make_optimizer(model):
                       lr=5e-5, betas=(0.9, 0.98), model=model)
 
 
+def dump_outputs(path, model, logits, loss, inference):
+    """What the timed step hands its caller, as path/<name>.npy (float32): the clip logits, and for a training step the loss and
+    a fixed, seeded sample of the gradients - every trainable parameter in named_parameters() order, all of its elements up to
+    1024, else max(1024, numel // 32) indices drawn from torch.Generator().manual_seed(0) (about 20 MB for ClipBERT's 149 M)."""
+    import numpy as np
+    out = dict(logits=torch.stack(logits) if isinstance(logits, (list, tuple)) else logits)
+    if not inference:
+        out["loss"] = loss
+        g = torch.Generator().manual_seed(0)
+        parts = []
+        for _, p_ in model.named_parameters():
+            if not p_.requires_grad:
+                continue
+            flat = p_.grad.reshape(-1)
+            if flat.numel() > 1024:
+                flat = flat[torch.randint(0, flat.numel(), (max(1024, flat.numel() // 32),), generator=g).to(flat.device)]
+            parts.append(flat.float())
+        out["grads"] = torch.cat(parts)
+    os.makedirs(path, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(path, name + ".npy"), v.detach().float().cpu().numpy())
+    return {name: tuple(v.shape) for name, v in out.items()}
+
+
 def lse_loss(logits_per_clip, labels):
     """Clip aggregation + loss of the reference loop (run_video_retrieval.py:404-422, pool_method 'lse')."""
     lg = (logits_per_clip if torch.is_tensor(logits_per_clip) else torch.stack(logits_per_clip)).permute(1, 0, 2).contiguous()
@@ -284,6 +308,9 @@ def run_b200(args):
     dbuf = {k: torch.empty(v.shape, dtype=v.dtype, device=dev) for k, v in host.items()}
     loss_host = _pin(torch.zeros(1, dtype=torch.float32))
     loss_dev = torch.zeros(1, dtype=torch.float32, device=dev)
+    # logits of the latest fwd_bwd (under graph replay the captured, static output of every replay), detached and cleared
+    # before the capture: a pass's autograd graph or buffers kept past its step and freed inside the capture break it
+    last = {}
 
     def h2d():
         for k in host:
@@ -296,6 +323,7 @@ def run_b200(args):
                 mb = dict(text_input_ids=dbuf["text_input_ids"], text_input_mask=dbuf["text_input_mask"], n_examples_list=[n_ex] * B)
                 logits = model.forward_clips(mb, n_clips, grid=grid)["logits"]
                 loss_dev.copy_(logits.float().mean().reshape(1))          # the per-step result read back by the e2e leg
+            last["logits"] = logits.detach()
             return
         if args.clip_batching:     # SURVEY §8 f1: the n_clips passes of the reference loop as ONE pass over B*n_clips units
             mb = dict(visual_inputs=dbuf["visual_inputs"], text_input_ids=dbuf["text_input_ids"], text_input_mask=dbuf["text_input_mask"],
@@ -311,6 +339,7 @@ def run_b200(args):
                 mb = dict(visual_inputs=vis[:, c], text_input_ids=dbuf["text_input_ids"], text_input_mask=dbuf["text_input_mask"],
                           labels=dbuf["labels"] if args.head == "retrieval" else None, n_examples_list=[n_ex] * B)
                 logits.append(model(mb)["logits"])
+        last["logits"] = logits.detach() if torch.is_tensor(logits) else [lg.detach() for lg in logits]
         loss = cb.clip_lse_loss(logits, dbuf["labels"]) if args.fused_loss else lse_loss(logits, dbuf["labels"])
         loss.backward()
         if world > 1:
@@ -397,6 +426,7 @@ def run_b200(args):
             torch.cuda.synchronize()
             g = torch.cuda.CUDAGraph()
             model.zero_grad()
+            last.clear()
             lc0 = ops.launch_count()
             with torch.cuda.graph(g, stream=s):
                 fwd_bwd()
@@ -452,6 +482,9 @@ def run_b200(args):
             ms_e2e = None
     if ms_e2e is None:
         ms_e2e, _, _ = timed(step_e2e, args.steps, max(3, args.warmup // 2))
+    if args.dump_outputs and rank == 0:      # the last timed step's results, before the untimed passes below overwrite them
+        shapes = dump_outputs(args.dump_outputs, model, last["logits"], loss_dev, args.inference)
+        print("[bench] outputs of the last timed step written to %s: %s" % (args.dump_outputs, shapes), file=sys.stderr)
     if graph is not None:          # kernels replayed from the captured graph do not pass through the C-ABI counter
         launches += captured_launches * args.steps
 
@@ -671,9 +704,9 @@ def run_reference(args):
         return
     b = args.cpu_batch
     sd, batch = _cpu_setup(args, b)
-    for _ in range(max(1, min(args.warmup, 1))):
+    for _ in range(args.warmup):
         _cpu_step(sd, batch, args.n_clips, args.n_frm, args.size)
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     t0 = time.time()
     for _ in range(steps):
         _cpu_step(sd, batch, args.n_clips, args.n_frm, args.size)
@@ -681,7 +714,7 @@ def run_reference(args):
     val = round(b * args.n_clips / dt, 3)
     L = args.txt_len + (args.size // 32 // 2) ** 2
     out = dict(impl="reference", metric=METRIC_TRAIN, value=val, unit="clips/s", n_gpus=args.gpus,
-               steps=steps, warmup=1, ms_per_step=round(dt * 1e3, 2), higher_is_better=True, scaling="weak", vs_baseline=None, dtype="f32",
+               steps=steps, warmup=args.warmup, ms_per_step=round(dt * 1e3, 2), higher_is_better=True, scaling="weak", vs_baseline=None, dtype="f32",
                data="synthetic",
                config=dict(workload="MSRVTT retrieval train step (bounded CPU sample): %d videos x %d clips x %d frames %dx%d, %d-token text, n_ex=%d"
                            % (b, args.n_clips, args.n_frm, args.size, args.size, args.txt_len, args.n_ex), seq_len=L,
@@ -696,8 +729,8 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 20; 3 with --impl reference, whose fp32 CPU steps take seconds)")
+    ap.add_argument("--warmup", type=int, default=None, help="untimed steps before them (default 5; 1 with --impl reference)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="headline", choices=sorted(CONFIGS), help="BASELINE.json workload (default: the configuration the metric names)")
     ap.add_argument("--batch", type=int, default=None, help="videos per GPU (default: the config's)")
@@ -736,7 +769,18 @@ def main():
     ap.add_argument("--optimizer", type=int, default=1, help="also time the fused AdamW step (informational key fused_optimizer)")
     ap.add_argument("--opt_steps", type=int, default=10, help="timed iterations of the informational fused-optimizer leg")
     ap.add_argument("--no_cpu", type=int, default=0, help="skip the CPU baseline leg (profiling runs)")
-    args = apply_config(ap.parse_args())
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (logits, loss, sampled gradients) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 3 if args.impl == "reference" else 20
+    if args.warmup is None:
+        args.warmup = 1 if args.impl == "reference" else 5
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of this repository's timed path; --impl reference has none to write")
+    args = apply_config(args)
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -3,8 +3,8 @@ may import this; the product path is clipbert_b200/optim.py + csrc/optim.cu).
 
 Follows src/optimization/adamw.py:40-103 (HuggingFace AdamW with the weight-decay fix) and
 torch.nn.utils.clip_grad_norm_ as called at src/tasks/run_video_retrieval.py:477-480. Pinned against the reference's
-own class (live import in tests/test_oracle.py where /root/reference exists) and tests/golden/adamw.pt generated from
-it by tools/make_golden_adamw.py.
+own class by tests/test_oracle.py, through tests/golden/adamw.pt and tests/golden/reference_live.pt generated from it by
+tools/make_golden_adamw.py and tools/make_golden_reference.py.
 """
 import math
 

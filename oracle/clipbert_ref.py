@@ -5,9 +5,9 @@ this module, and only as the checker / the CPU arm; the product path (clipbert_b
 
 Pinning status
   * Transformer half (a9-a21): restated here in plain functional PyTorch fp32 and PINNED against the
-    reference's own code — /root/reference/src/modeling/{modeling,transformers}.py imported through
-    oracle/ref_import.py — by tests/test_oracle.py (runs where /root/reference exists) and by the
-    golden vectors under tests/golden/ that tools/make_golden.py generated from that import.
+    reference's own code — src/modeling/{modeling,transformers}.py imported through oracle/ref_import.py —
+    by tests/test_oracle.py, against the golden vectors under tests/golden/ that tools/make_golden.py and
+    tools/make_golden_reference.py generated from that import.
   * CNN half (a2-a7): the arithmetic lives in detectron2 @ ffff8ac (docker/Dockerfile:13), which is
     NOT vendored in /root/reference and not installable offline. Restated from the published d2
     algorithm (modeling/backbone/resnet.py: BasicStem, BottleneckBlock with STRIDE_IN_1X1=True;

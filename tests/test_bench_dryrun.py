@@ -54,12 +54,11 @@ def _ctx(*a, **k):
     yield
 
 
-@pytest.mark.parametrize("flags", [["--graph", "1", "--size", "128"],
-                                   ["--graph", "0", "--prefetch", "0", "--fused_loss", "1", "--recast_in_step", "1", "--clip_batching", "0",
-                                    "--stem", "im2col", "--mn3d", "1", "--occ2", "2"]])
-def test_bench_control_flow_on_cpu(monkeypatch, capsys, flags):
+@pytest.fixture
+def bench_on_cpu(monkeypatch):
+    """bench.py in this process, single rank, with torch.cuda's streams / events / graphs replaced by the inert stand-ins above
+    and the device set to the CPU (the C-ABI calls are answered by ops_emulator.emulated_ops in each test)."""
     import bench
-    from ops_emulator import emulated_ops
     cpu = torch.device("cpu")
     for name, val in (("Stream", _Stream), ("Event", _Event), ("CUDAGraph", _Graph), ("graph", _ctx), ("stream", _ctx),
                       ("current_stream", lambda *a: _Stream()), ("synchronize", lambda *a: None), ("set_device", lambda *a: None),
@@ -67,12 +66,21 @@ def test_bench_control_flow_on_cpu(monkeypatch, capsys, flags):
         monkeypatch.setattr(torch.cuda, name, val)
     monkeypatch.setattr(bench, "_device", lambda r: cpu)
     monkeypatch.setattr(bench, "_pin", lambda t: t)
+    for k in ("RANK", "LOCAL_RANK", "WORLD_SIZE"):
+        monkeypatch.delenv(k, raising=False)
+    return bench
+
+
+@pytest.mark.parametrize("flags", [["--graph", "1", "--size", "128"],
+                                   ["--graph", "0", "--prefetch", "0", "--fused_loss", "1", "--recast_in_step", "1", "--clip_batching", "0",
+                                    "--stem", "im2col", "--mn3d", "1", "--occ2", "2"]])
+def test_bench_control_flow_on_cpu(bench_on_cpu, monkeypatch, capsys, flags):
+    bench = bench_on_cpu
+    from ops_emulator import emulated_ops
     argv = ["bench.py", "--gpus", "1", "--steps", "2", "--warmup", "1", "--batch", "2", "--n_clips", "2", "--n_frm", "1", "--size", "64",
             "--txt_len", "12", "--no_cpu", "1", "--overlap_wgrad", "0", "--opt_steps", "1"] + flags
     size = int(flags[flags.index("--size") + 1]) if "--size" in flags else 64
     monkeypatch.setattr(sys, "argv", argv)
-    for k in ("RANK", "LOCAL_RANK", "WORLD_SIZE"):
-        monkeypatch.delenv(k, raising=False)
     with emulated_ops(ignore_dropout=True) as calls:
         bench.main()
     out, err = capsys.readouterr()
@@ -100,24 +108,15 @@ def test_bench_control_flow_on_cpu(monkeypatch, capsys, flags):
 
 
 @pytest.mark.parametrize("config", ["c4", "c5"])
-def test_bench_other_baseline_configs_on_cpu(monkeypatch, capsys, config):
+def test_bench_other_baseline_configs_on_cpu(bench_on_cpu, monkeypatch, capsys, config):
     """bench.py --config c4 (TGIF-QA multiple choice train step) and c5 (paragraph-retrieval inference: CNN once per video, one
     BERT pass over clips x captions) in miniature through the emulated ABI: the workload plumbing and the JSON line."""
-    import bench
+    bench = bench_on_cpu
     from ops_emulator import emulated_ops
-    cpu = torch.device("cpu")
-    for name, val in (("Stream", _Stream), ("Event", _Event), ("CUDAGraph", _Graph), ("graph", _ctx), ("stream", _ctx),
-                      ("current_stream", lambda *a: _Stream()), ("synchronize", lambda *a: None), ("set_device", lambda *a: None),
-                      ("is_available", lambda: False)):
-        monkeypatch.setattr(torch.cuda, name, val)
-    monkeypatch.setattr(bench, "_device", lambda r: cpu)
-    monkeypatch.setattr(bench, "_pin", lambda t: t)
     small = {"c4": ["--batch", "2", "--n_ex", "3", "--txt_len", "12"], "c5": ["--n_clips", "3", "--n_ex", "2", "--txt_len", "70"]}[config]
     argv = ["bench.py", "--config", config, "--gpus", "1", "--steps", "2", "--warmup", "1", "--size", "64", "--no_cpu", "1", "--overlap_wgrad", "0",
             "--opt_steps", "1", "--graph", "0", "--prefetch", "0"] + small
     monkeypatch.setattr(sys, "argv", argv)
-    for k in ("RANK", "LOCAL_RANK", "WORLD_SIZE"):
-        monkeypatch.delenv(k, raising=False)
     with emulated_ops(ignore_dropout=True) as calls:
         bench.main()
     out, err = capsys.readouterr()
@@ -130,6 +129,84 @@ def test_bench_other_baseline_configs_on_cpu(monkeypatch, capsys, config):
     else:
         assert "inference" in d["metric"] and d["config"]["clips_per_step_per_gpu"] == 3 and d["config"]["seq_len"] == 71
         assert d["fused_optimizer"] is None and calls["attention_bwd"] == 0 and calls["attention_fwd"] > 0
+
+
+@pytest.mark.parametrize("graph", ["0", "1"])
+def test_bench_dump_outputs_on_cpu(bench_on_cpu, monkeypatch, capsys, tmp_path, graph):
+    """--dump-outputs DIR: after the timed steps the logits, loss and a seeded sample of the gradients of the last step land in
+    DIR as float32 .npy files, under 64 MB, the loss is the one of those logits, and two runs with the same arguments write the
+    same arrays. (The stand-in graph replays nothing, so this checks the plumbing; the GPU test below runs the real graph.)"""
+    import types
+    import numpy as np
+    bench = bench_on_cpu
+    from ops_emulator import emulated_ops
+    runs = []
+    for i in range(2):
+        out = tmp_path / ("run%d" % i)
+        monkeypatch.setattr(sys, "argv", ["bench.py", "--gpus", "1", "--steps", "2", "--warmup", "1", "--batch", "2", "--n_clips", "2",
+                                          "--n_frm", "1", "--size", "64", "--txt_len", "12", "--no_cpu", "1", "--overlap_wgrad", "0",
+                                          "--opt_steps", "1", "--graph", graph, "--dump-outputs", str(out)])
+        with emulated_ops(ignore_dropout=True):
+            bench.main()
+        capsys.readouterr()
+        runs.append({f.name[:-4]: np.load(str(f)) for f in sorted(out.iterdir())})
+    a, b = runs
+    assert sorted(a) == ["grads", "logits", "loss"]
+    assert a["logits"].shape == (2, 2, 2) and a["loss"].shape == (1,) and all(v.dtype == np.float32 for v in a.values())
+    assert a["grads"].size > 100e6 / 32 and sum(v.nbytes for v in a.values()) <= 64 << 20     # 1/32 of > 100 M gradients
+    assert np.isfinite(a["grads"]).all() and np.abs(a["grads"]).max() > 0
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k
+    labels = bench.make_host_batch(types.SimpleNamespace(batch=2, n_clips=2, n_frm=1, size=64, n_ex=1, txt_len=12, head="retrieval"), 0)["labels"]
+    assert abs(float(bench.lse_loss(torch.from_numpy(a["logits"]), labels)) - float(a["loss"][0])) < 1e-5
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_with_the_cuda_graph_on_the_device(cuda, tmp_path):
+    """bench.py --dump-outputs on the device, whole-step CUDA graph on: the graph is used, the dumped loss is the LSE loss of the
+    dumped logits (both from one replay), and one more timed step changes what is written - dropout draws fresh masks at every
+    replay - so the arrays come from the timed steps, not from the capture."""
+    import subprocess
+    import types
+    import numpy as np
+    import bench
+    env = {k: v for k, v in os.environ.items() if k not in ("RANK", "LOCAL_RANK", "WORLD_SIZE")}
+    runs = {}
+    for steps in (3, 4):
+        out = tmp_path / ("steps%d" % steps)
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", "2", "--batch", "4",
+                            "--no_cpu", "1", "--opt_steps", "1", "--dump-outputs", str(out)], capture_output=True, text=True, env=env, timeout=900)
+        assert r.returncode == 0, r.stderr[-3000:]
+        d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+        assert d["steps"] == steps and d["config"]["cuda_graph"] is True and "capture failed" not in r.stderr, r.stderr[-3000:]
+        runs[steps] = {f.name[:-4]: np.load(str(f)) for f in sorted(out.iterdir())}
+    args = types.SimpleNamespace(batch=4, n_clips=2, n_frm=2, size=224, n_ex=1, txt_len=32, head="retrieval")
+    labels = bench.make_host_batch(args, 0)["labels"]
+    for a in runs.values():
+        assert sorted(a) == ["grads", "logits", "loss"] and a["logits"].shape == (2, 4, 2)
+        assert np.isfinite(a["grads"]).all() and np.abs(a["grads"]).max() > 0
+        want = float(bench.lse_loss(torch.from_numpy(a["logits"]).double(), labels))
+        assert abs(want - float(a["loss"][0])) < 1e-4 * max(1.0, abs(want)), (want, a["loss"])
+    assert not np.array_equal(runs[3]["logits"], runs[4]["logits"]) and not np.array_equal(runs[3]["grads"], runs[4]["grads"])
+
+
+@pytest.mark.parametrize("flags,steps,warmup",[(["--steps", "4", "--warmup", "0"], 4, 0), ([], 3, 1)])
+def test_bench_reference_arm_times_the_steps_asked_for(bench_on_cpu, monkeypatch, capsys, flags, steps, warmup):
+    """--impl reference (the CPU oracle) runs exactly --warmup untimed and --steps timed steps (defaults 1 and 3 there) and reports
+    them; --dump-outputs, which writes the outputs of this repository's timed path, is refused with it."""
+    bench = bench_on_cpu
+    calls = []
+    real = bench._cpu_step
+    monkeypatch.setattr(bench, "_cpu_step", lambda *a: calls.append(1) or real(*a))
+    base = ["bench.py", "--impl", "reference", "--cpu_batch", "1", "--n_clips", "1", "--n_frm", "1", "--size", "64", "--txt_len", "12"]
+    monkeypatch.setattr(sys, "argv", base + flags)
+    bench.main()
+    d = json.loads([l for l in capsys.readouterr().out.splitlines() if l.startswith("{")][-1])
+    assert d["impl"] == "reference" and d["steps"] == steps and d["warmup"] == warmup and len(calls) == steps + warmup
+    monkeypatch.setattr(sys, "argv", base + ["--dump-outputs", "unused"])
+    with pytest.raises(SystemExit) as e:
+        bench.main()
+    assert e.value.code == 2 and "--dump-outputs" in capsys.readouterr().err
 
 
 def calls_per_step_expected(flags):

@@ -1,27 +1,15 @@
 """CPU tests of the checkpoint key-layout helpers (SURVEY §8 f4, clipbert_b200/load_save.py) - index/key work, so the
-bar is exact equality. Where /root/reference exists the reference's own two functions are executed (their source is cut out
-of src/utils/load_save.py with ast - the module itself imports apex / easydict) and compared key for key."""
-import ast
+bar is exact equality. What the reference's own two functions (src/utils/load_save.py) do with the same inputs is stored in
+tests/golden/reference_helpers.json (tools/make_golden_reference.py) and compared key for key."""
+import json
 import os
-import types
 
 import pytest
 import torch
 
 from util import make_cfg
 
-REF = os.path.join(os.environ.get("CLIPBERT_REFERENCE_ROOT", "/root/reference"), "src", "utils", "load_save.py")
-
-
-def _reference_functions():
-    src = open(REF).read()
-    tree = ast.parse(src)
-    wanted = {"load_state_dict_with_mismatch", "convert_torchvision_ckpt_to_detectron2"}
-    body = [n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name in wanted]
-    ns = {"torch": torch, "os": os, "Dict": dict, "Any": object, "Union": object,
-          "LOGGER": types.SimpleNamespace(info=lambda *a, **k: None)}
-    exec(compile(ast.Module(body=body, type_ignores=[]), REF, "exec"), ns)
-    return ns
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_helpers.json")
 
 
 def _model():
@@ -86,24 +74,24 @@ def test_load_state_dict_with_mismatch_skips_foreign_and_misshapen_keys_and_roun
     assert all(torch.equal(a, b) for a, b in zip(fresh.state_dict().values(), model.state_dict().values()))
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="needs /root/reference")
 def test_helpers_agree_with_the_reference_functions(tmp_path):
     from clipbert_b200 import load_save as LS
-    ref = _reference_functions()
+    gold = json.load(open(GOLD))
     tv = _tv_resnet50_state_dict()
     path = str(tmp_path / "tv.pth")
     torch.save(tv, path)
-    want = ref["convert_torchvision_ckpt_to_detectron2"](path)
     got = LS.convert_torchvision_ckpt_to_detectron2(path)
-    assert list(got["model"].keys()) == list(want["model"].keys()) and got["matching_heuristics"] == want["matching_heuristics"]
-    assert all(torch.equal(got["model"][k], want["model"][k]) for k in want["model"])
-    # load_state_dict_with_mismatch: run the reference's function and ours on two copies of the transformer
+    # the reference's output: these detectron2 names, in this order, each holding the torchvision tensor named beside it
+    assert list(got["model"].keys()) == [d2 for d2, _ in gold["d2_key_map"]]
+    assert got["matching_heuristics"] == gold["d2_matching_heuristics"]
+    assert all(torch.equal(got["model"][d2], tv[src]) for d2, src in gold["d2_key_map"])
+    # load_state_dict_with_mismatch: ours against the transformer the reference's function leaves (it loads exactly these keys)
     from oracle import synth
     sd = {k[len("transformer."):]: v for k, v in synth.full_state_dict(7).items() if k.startswith("transformer.")}
     sd["classifier.2.weight"] = torch.zeros(7, 1536)
     sd["extra.weight"] = torch.zeros(3)
     a, b = _model().transformer, _model().transformer
-    ref["load_state_dict_with_mismatch"](a, sd)
+    a.load_state_dict({k: sd[k] for k in gold["mismatch_loaded_keys"]}, strict=False)
     LS.load_state_dict_with_mismatch(b, sd)
     assert all(torch.equal(x, y) for x, y in zip(a.state_dict().values(), b.state_dict().values()))
 
